@@ -1,6 +1,6 @@
-"""Reference arm of bench.py: the UNMODIFIED reference modules (baseline/_ref/learning/*, copied
-verbatim from /root/reference by install_ref.py) driven through their own public API on the host
-CPU — pointnet.PointNet / CloudEmbedder.run, graphnet.GraphNetwork (use_pyg=0, cuda=False: the
+"""Reference arm of bench.py: the UNMODIFIED reference modules (learning/*, compiled to oracle/_ref/ by
+oracle/build_ref.py) driven through their own public API on the host CPU —
+pointnet.PointNet / CloudEmbedder.run, graphnet.GraphNetwork (use_pyg=0, cuda=False: the
 reference's own CPU code path incl. the per-node loops of ecc/GraphConvModule.py:82-88,114-121),
 ecc.GraphConvInfo, cross entropy, element-wise clamp, torch.optim.Adam (learning/main.py:199-213;
 eval: main.py:229-264).  None of this repository's kernels, modules or oracle is on this path.
@@ -16,12 +16,13 @@ from types import SimpleNamespace
 
 import torch
 
-HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.path.join(HERE, "_ref")
+from oracle import build_ref
+
+REF = build_ref.DST
 
 
 def available():
-    return os.path.exists(os.path.join(REF, "learning", "pointnet.py"))
+    return build_ref.available()
 
 
 def _import():

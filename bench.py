@@ -20,11 +20,14 @@ Timing: every step is bracketed by CUDA events on the launching stream; an L2 fl
 memset) runs between steps outside the brackets; the reported time is the max over ranks of the
 summed step times, after a barrier + synchronize on both sides of the K steps.
 
-Reference arm: baseline/_ref/ holds a verbatim copy of the reference's learning/{pointnet,graphnet,
-modules}.py and learning/ecc/* (baseline/install_ref.py, run by __graft_entry__.build() where
-/root/reference exists; git-ignored, shipped with the snapshot).  `--impl reference` drives those
-modules through their own API on the host CPU (baseline/ref_arm.py); `cpu_baseline.kind` is
-"reference" then, "port" (oracle/nets_ref) only if the copy is missing.
+Reference arm: build() compiles the reference's learning/{pointnet,graphnet,modules}.py and
+learning/ecc/* to bytecode under oracle/_ref/ where a reference checkout exists (oracle/build_ref.py).
+`--impl reference` drives those modules through their own API on the host CPU (baseline/ref_arm.py);
+`cpu_baseline.kind` is "reference" then, "port" (oracle/nets_ref) without them.
+
+`--dump-outputs DIR` writes what the timed path returned in its last timed step (rank 0): logits.npy
+(float32 [superpoints, classes]) and, for training workloads, loss.npy (float32 [1]).  Inputs and
+initial weights are seeded, so two builds run with the same arguments can be compared array by array.
 """
 import argparse
 import json
@@ -62,7 +65,12 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer pass (profiling runs)")
     ap.add_argument("--trace-gemm", action="store_true", help="per-shape timing of the SIMT GEMM calls (stderr)")
     ap.add_argument("--no-graph", action="store_true", help="time eager launches only (no CUDA-graph replay)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (float32, at most 64 MB in all)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
 
 
 def peaks():
@@ -188,8 +196,8 @@ def host_info():
 
 
 class CpuArm(object):
-    """The reference's CPU path for one workload: the reference's OWN modules when baseline/_ref is
-    installed (kind "reference": baseline/ref_arm.py), else the oracle port (kind "port")."""
+    """The reference's CPU path for one workload: the reference's OWN modules when oracle/_ref holds
+    them (kind "reference": baseline/ref_arm.py), else the oracle port (kind "port")."""
 
     def __init__(self, w, sd_ecc=None, sd_ptn=None):
         from baseline import ref_arm
@@ -243,7 +251,7 @@ class CpuArm(object):
         if getattr(self, "note", None):
             return "oracle port of the reference CPU path (oracle/nets_ref, ecc_mode=loop); " + self.note
         if self.kind == "reference":
-            return ("the reference's own modules (baseline/_ref: learning/pointnet.py, graphnet.py, modules.py, "
+            return ("the reference's own modules (oracle/_ref: learning/pointnet.py, graphnet.py, modules.py, "
                     "ecc/*; use_pyg=0, cuda=False) through CloudEmbedder.run / GraphNetwork / cross_entropy / "
                     "clamp / Adam")
         return "oracle port of the reference CPU path (oracle/nets_ref, ecc_mode=loop)"
@@ -503,6 +511,32 @@ def loader_roofline(dev, pk, with_cpu):
     return out
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def host_outputs(loss, logits):
+    """A step's (loss, logits) as float32 host arrays, copied now: a replayed graph reuses its output buffers."""
+    out = {"logits": logits.detach().float().cpu().numpy()}
+    if loss is not None:
+        out["loss"] = loss.detach().float().reshape(-1).cpu().numpy()
+    return out
+
+
+def dump_outputs(path, arrays, budget=DUMP_BYTES):
+    """Writes every array as path/<name>.npy.  Past `budget` bytes in all, logits keeps a fixed seeded
+    sample of its rows, whose indices go to logits_rows.npy (float64)."""
+    arrays = dict(arrays)
+    lg = arrays["logits"]
+    rest = sum(a.nbytes + 128 for k, a in arrays.items() if k != "logits") + 2 * 128  # + .npy headers
+    if rest + lg.nbytes > budget:
+        keep = (budget - rest) // (lg.shape[1] * lg.itemsize + 8)
+        rows = np.sort(np.random.default_rng(0).choice(lg.shape[0], keep, replace=False))
+        arrays["logits"], arrays["logits_rows"] = lg[rows], rows.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def run_b200(args):
     import torch.distributed as dist
 
@@ -578,13 +612,14 @@ def run_b200(args):
         flush.zero_()  # L2 flush, outside the event bracket
         s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         s.record()
-        step(dbs[i % nb])
+        out = step(dbs[i % nb])
         e.record()
         evs.append((s, e))
         done_units += units[i % nb]
     barrier()
     wall = time.perf_counter() - t_wall
     clocks = sampler.stop()
+    last = host_outputs(*out) if args.dump_outputs else None
     launches = ops.total_launches() - launches0
     total_ms = sum(s.elapsed_time(e) for s, e in evs)
     tt = torch.tensor([total_ms], dtype=torch.float64, device=dev)
@@ -615,7 +650,7 @@ def run_b200(args):
                 flush.zero_()
                 s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 s.record()
-                trainer.replay(graph_keys[i % nb])
+                out = trainer.replay(graph_keys[i % nb])
                 e.record()
                 evs.append((s, e))
                 done_units += units[i % nb]
@@ -631,6 +666,8 @@ def run_b200(args):
                 dist.all_reduce(uu, op=dist.ReduceOp.SUM)
             total_ms, all_units = float(tt), float(uu)
             value = all_units / (total_ms * 1e-3)
+            if args.dump_outputs:
+                last = host_outputs(*out)
         except Exception as ex:  # keep the eager numbers
             graph_keys, graph_err = None, repr(ex)
     eval_keys = None
@@ -652,7 +689,7 @@ def run_b200(args):
                 flush.zero_()
                 s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 s.record()
-                trainer.replay_eval(eval_keys[i % nb])
+                out = None, trainer.replay_eval(eval_keys[i % nb])
                 e.record()
                 evs.append((s, e))
                 done_units += units[i % nb]
@@ -668,6 +705,8 @@ def run_b200(args):
                 dist.all_reduce(uu, op=dist.ReduceOp.SUM)
             total_ms, all_units = float(tt), float(uu)
             value = all_units / (total_ms * 1e-3)
+            if args.dump_outputs:
+                last = host_outputs(*out)
         except Exception as ex:  # keep the eager numbers
             eval_keys, graph_err = None, repr(ex)
 
@@ -833,6 +872,8 @@ def run_b200(args):
             print("[gemm_f32] %-40s x%d  %.3f ms" % (desc, n, ms), file=sys.stderr)
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         line["cpu_baseline"] = cpu_baseline(w, sd_ecc, sd_ptn)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
     if rank == 0:
         print(json.dumps(line))
     if world > 1:

@@ -6,8 +6,8 @@
   names (learning.pointnet / graphnet / modules / ecc) before main.py's imports run;
 * packages the image lacks (igraph, h5py, torchnet, transforms3d) resolve to the stand-ins in this
   directory — only if the real ones cannot be imported;
-* main.py itself is executed with runpy from the reference checkout (default: /root/reference, else the
-  verbatim copy under baseline/_ref), byte for byte as it lies there.
+* main.py itself is executed with runpy, unmodified: from the checkout given by --reference-root, else
+  as the bytecode oracle/build_ref.py compiled from the reference into oracle/_ref/.
 """
 import importlib
 import os
@@ -33,11 +33,21 @@ def _use_standins():
     return missing
 
 
+def main_script(ref):
+    """learning/main.py of a checkout, or learning/main.pyc of oracle/_ref; None if there is neither."""
+    for name in ("main.py", "main.pyc"):
+        path = os.path.join(ref, "learning", name)
+        if os.path.exists(path):
+            return path
+    return None
+
+
 def reference_root(explicit=None):
-    for cand in (explicit, os.environ.get("SPG_REFERENCE"), "/root/reference", os.path.join(ROOT, "baseline", "_ref")):
-        if cand and os.path.exists(os.path.join(cand, "learning", "main.py")):
+    for cand in (explicit, os.path.join(ROOT, "oracle", "_ref")):
+        if cand and main_script(cand):
             return cand
-    raise RuntimeError("no reference checkout with learning/main.py found (run baseline/install_ref.py)")
+    raise RuntimeError("no reference learning/main.py found (pass --reference-root, or build oracle/_ref with "
+                       "python -m oracle.build_ref)")
 
 
 def run(main_args, ref_root=None):
@@ -53,7 +63,7 @@ def run(main_args, ref_root=None):
         sys.path.remove(learning_dir)
     sys.path.insert(0, learning_dir)
     old_argv = sys.argv
-    sys.argv = [os.path.join(learning_dir, "main.py")] + list(main_args)
+    sys.argv = [main_script(ref)] + list(main_args)
     try:
         print("[run_main] reference: %s  stand-ins: %s" % (ref, ", ".join(standins) or "none"), flush=True)
         runpy.run_path(sys.argv[0], run_name="__main__")

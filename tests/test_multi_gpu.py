@@ -66,7 +66,7 @@ def _worker(rank, world, port, q):
     dist.destroy_process_group()
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 def test_fused_allreduce_adam_matches_nccl_path_world2():
     import torch.multiprocessing as mp
     ctx = mp.get_context("spawn")
