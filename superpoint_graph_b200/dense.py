@@ -149,6 +149,10 @@ def chain_forward(inp, M, specs, params, training, saved=None):
         else:
             res = ops.gemm(cur.raw, cur.ld, True, W, sp.cin, True, M, sp.cout, sp.cin, bias=bias,
                            a_aff=cur.aff(), stats=batch_stats, fold=fold)
+        if fold is not None and fold[3] is not None:
+            # the kernel updated the running statistics in place: tell torch, so that caches keyed on
+            # version counters (ops.pointnet_fused_image) see the change
+            torch.autograd.graph.increment_version([fold[3], fold[4], fold[5]])
         mean = var = scale = shift = None
         y = res
         if bn is not None:

@@ -5,6 +5,7 @@ on torch's current stream.  CPU tensors are rejected: there is no CPU implementa
 product (the CPU restatement lives in oracle/ and is test infrastructure only).
 """
 import os
+import weakref
 
 import numpy as np
 import torch
@@ -873,24 +874,32 @@ def pointnet_fused_supported(F, L, widths):
     return USE_FUSED_EVAL[0] and bool(_lib.lib().spg_pointnet_fused_supported(int(F), int(L), len(widths), w.data_ptr()))
 
 
-_FUSED_IMAGES = {}  # parameter versions -> (weight image, folded bias, widths tensor)
+_FUSED_IMAGES = {}  # parameter versions -> (weight image, folded bias, widths tensor, weakrefs to the sources)
 EVAL_BF16 = [False]  # eval-mode PointNet trunk in bf16 arithmetic (Trainer(dtype="bf16") sets it around eval_step)
+
+
+def _root(t):
+    return t if t._base is None else t._base
 
 
 def pointnet_fused_image(layers, F, bf16=False):
     """layers: [(W [N,K] (2-D view), bias|None, bn_module|None)] of a Conv1d(k=1)+BatchNorm+ReLU chain in eval
     mode.  Returns (image, bias, widths): BatchNorm folded into weights and bias (scale = gamma/sqrt(rv+eps),
     bias' = bias*scale + beta - rm*scale), packed for spg_pointnet_fused_eval (fp32: tf32 hi|lo blocks of 32
-    floats) or spg_pointnet_fused_eval_bf16 (bf16 blocks of 64 elements).  Cached on the tensors' version
-    counters (eval weights do not change between batches)."""
-    key = []
+    floats) or spg_pointnet_fused_eval_bf16 (bf16 blocks of 64 elements).  Cached on the tensors' addresses and
+    version counters (eval weights do not change between batches).  Whoever writes these tensors behind
+    torch's back (the Trainer's optimizer kernel, the running-statistics update of a training forward) bumps
+    their version counters.  An entry also holds weak references to its source tensors: a tensor that died, or
+    a different tensor at a recycled address with an equal version count, is a miss."""
+    key, srcs = [], []
     for W, b, bn in layers:
         ts = [W, b] + ([bn.running_mean, bn.running_var, bn.weight, bn.bias] if bn is not None else [])
         key += [(x.data_ptr(), x._version) for x in ts if x is not None]
+        srcs += [_root(x) for x in ts if x is not None]
     key = (int(F), bool(bf16)) + tuple(key)
     ent = _FUSED_IMAGES.get(key)
-    if ent is not None:
-        return ent
+    if ent is not None and all(r() is x for r, x in zip(ent[3], srcs)):
+        return ent[:3]
     dev = layers[0][0].device
     L = _lib.lib()
     widths = torch.tensor([int(W.shape[0]) for W, _, _ in layers], dtype=torch.int32)
@@ -928,7 +937,7 @@ def pointnet_fused_image(layers, F, bf16=False):
         K = max(N, kc) if bf16 else N
     if len(_FUSED_IMAGES) > 64:
         _FUSED_IMAGES.clear()
-    _FUSED_IMAGES[key] = (image, bias, widths)
+    _FUSED_IMAGES[key] = (image, bias, widths, [weakref.ref(x) for x in srcs])
     return image, bias, widths
 
 

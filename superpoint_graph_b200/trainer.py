@@ -130,6 +130,7 @@ class Trainer(object):
         self.exp_avg = torch.zeros_like(self.flat)
         self.exp_avg_sq = torch.zeros_like(self.flat)
         self.step_count = 0
+        self._generation = 0  # bumped whenever the parameters change (see _params_changed)
         self._learned_packs = {}  # weight images packed on demand by earlier steps (see compute_gradients)
         self._side = ops.SideStream(self.flat.device) if (self.flat.is_cuda and ops.USE_SIDE_STREAM[0]) else None
         self._capturing = False
@@ -217,11 +218,20 @@ class Trainer(object):
         if self._fused_ar is not None:
             self._fused_ar.step_(self.flat, self.exp_avg, self.exp_avg_sq, self.step_dev, lr=self.args.lr,
                                  weight_decay=self.args.wd, grad_clip=self.args.grad_clip)
-            return
-        self.reduce_gradients()
-        ops.clamp_adam_dev_(self.flat, self.flat_grad, self.exp_avg, self.exp_avg_sq, self.step_dev,
-                            lr=self.args.lr, weight_decay=self.args.wd, grad_clip=self.args.grad_clip,
-                            grad_scale=1.0 / self.world_size)
+        else:
+            self.reduce_gradients()
+            ops.clamp_adam_dev_(self.flat, self.flat_grad, self.exp_avg, self.exp_avg_sq, self.step_dev,
+                                lr=self.args.lr, weight_decay=self.args.wd, grad_clip=self.args.grad_clip,
+                                grad_scale=1.0 / self.world_size)
+        self._params_changed()
+
+    def _params_changed(self):
+        """The parameters were written through `flat`, behind torch's back.  Bump their version counters,
+        one per tensor (the parameters are views of `flat` with counters of their own): caches keyed on
+        versions (the folded eval weight images) then rebuild, and eval graphs captured before this point
+        refuse to replay."""
+        torch.autograd.graph.increment_version(self.params)
+        self._generation += 1
 
     def reduce_gradients(self):
         """The step's only collective: SUM of the flat gradient over the scene-parallel ranks (the
@@ -255,6 +265,7 @@ class Trainer(object):
         self.step_count = step_count
         for b, sv in zip(bufs, saved):
             b.copy_(sv)
+        self._params_changed()
 
     def capture(self, db, key=None, warmup=2):
         """Captures compute_gradients on the static tensors of `db`; returns the key for replay().
@@ -287,6 +298,8 @@ class Trainer(object):
     def replay(self, key):
         g, db, loss, logits = self._graphs[key]
         g.replay()
+        # the replayed forward updated the BatchNorm running statistics without running chain_forward's host code
+        torch.autograd.graph.increment_version(list(self.model.buffers()))
         self.apply_update()  # (NCCL path: outside the graph; fused path: one more kernel launch)
         return loss, logits
 
@@ -317,11 +330,16 @@ class Trainer(object):
                 logits = self.eval_step(db)
         finally:
             self._capturing = False
-        self._graphs[key] = (g, db, None, logits)
+        self._graphs[key] = (g, db, self._generation, logits)
         return key
 
     def replay_eval(self, key):
-        g, db, _, logits = self._graphs[key]
+        """Replays a capture_eval graph.  The graph holds the folded weight images of the parameters it was
+        captured with, so it refuses to run once an update changed them: capture again."""
+        g, db, generation, logits = self._graphs[key]
+        if generation != self._generation:
+            raise RuntimeError("replay_eval: the parameters changed since capture_eval (the graph would run the "
+                               "old weights); capture the inference forward again")
         g.replay()
         return logits
 
